@@ -17,6 +17,9 @@ utterance path; the packed weights are broadcast once from rank 0 over NCCL at i
   extra    : N = 1 only -- BASELINE configs[2] (64 utterances in one call) with its own roofline, configs[4] (2000-phoneme
              streaming: time to first chunk / total) and the fp32-exact mode (precision 0) of the headline workload.
   --impl reference : the CPU path (oracle restatement of the reference's PyTorch graph) on the host cores.
+  --dump-outputs DIR : after the timed steps, writes what the last timed step returned to its caller (DIR/wav.npy float32
+             [1, frames * 256], DIR/y_lengths.npy float64), so that two builds can be compared output for output on the
+             same seeded inputs and weights.
 """
 import argparse
 import json
@@ -407,7 +410,10 @@ def main():
     ap.add_argument("--cpu-steps", type=int, default=5)
     ap.add_argument("--precision", type=int, default=1, help="0: fp32 FFMA everywhere; 1: flow+decoder on tcgen05 (split-bf16 x3); 2: encoder too; 3: encoder on tcgen05 with the exact 3-way split")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary configs (configs[2], configs[4], fp32-exact mode)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     from vosk_tts_b200 import config as C
     cfg = C.DEFAULT_CONFIG
@@ -512,11 +518,15 @@ def main():
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(estream)
-        step_dev()
+        last_frames = step_dev()
         e1.record(estream)
         e1.synchronize()
         step_ms.append(e0.elapsed_time(e1))
     barrier()
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "wav.npy"), d_wav[:, : last_frames * hop].cpu().numpy().astype(np.float32))
+        np.save(os.path.join(args.dump_outputs, "y_lengths.npy"), np.array([last_frames], np.float64))
     launches = eng.kernel_launches() - launches0
     total_ms = float(sum(step_ms))
     # roofline pass: same steps with every conv launch bracketed by CUDA events on the engine stream (eager launches,

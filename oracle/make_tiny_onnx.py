@@ -1,9 +1,10 @@
-"""TEST INFRASTRUCTURE ONLY -- writes tests/golden/tiny_model.onnx + tests/golden/tiny_onnx.npz.
+"""TEST INFRASTRUCTURE ONLY -- writes tests/golden/tiny_model_onnx.npz + tests/golden/tiny_onnx.npz.
 
 A reduced-width VITS2 / MB-iSTFT model (same topology as the reference configuration, 64 instead of 192 channels, three
 encoder layers, two resblock kernels) is built from the UNMODIFIED reference classes, exported with the reference's own
 export recipe (training/vits2/onnx_export.py:60-104 via oracle/ref_harness.export_reference_onnx) and run once through
-``SynthesizerTrn.infer`` with injected noise.  The fixture lets the GPU box (no reference tree there) prove the
+``SynthesizerTrn.infer`` with injected noise.  The exported file is stored in the compact form of oracle/onnx_fixture.py
+(weights regenerated from the seed, exact bytes checked).  The fixture lets the GPU box (no reference tree there) prove the
 deployment path end to end: model.onnx -> initializers -> packed weights -> engine == reference output.
 
 Run in the build container:  python oracle/make_tiny_onnx.py
@@ -11,6 +12,7 @@ Run in the build container:  python oracle/make_tiny_onnx.py
 import copy
 import os
 import sys
+import tempfile
 
 import numpy as np
 import torch
@@ -18,7 +20,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
-from oracle import ref_harness as rh  # noqa: E402
+from oracle import onnx_fixture, ref_harness as rh  # noqa: E402
 from vosk_tts_b200 import config as C, synthetic  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
@@ -42,8 +44,10 @@ def main():
     sd = synthetic.make_random_checkpoint(cfg, 77)
     net = rh.build_reference_model(sd, cfg=tj, n_vocab=N_VOCAB)
     os.makedirs(OUT, exist_ok=True)
-    path = os.path.join(OUT, "tiny_model.onnx")
-    rh.export_reference_onnx(path, net, n_vocab=N_VOCAB)
+    with tempfile.TemporaryDirectory() as tmp:
+        path = rh.export_reference_onnx(os.path.join(tmp, "model.onnx"), net, n_vocab=N_VOCAB)
+        onnx_bytes = os.path.getsize(path)
+        onnx_fixture.pack(path, os.path.join(OUT, "tiny_model_onnx.npz"), cfg, 77)
     g = torch.Generator().manual_seed(5)
     T, sid, scales = 23, 3, [0.8, 1.0, 0.8]
     tok = torch.randint(0, N_VOCAB, (1, T), generator=g)
@@ -56,7 +60,7 @@ def main():
                         scales=np.asarray(scales, np.float32), eps_dp=eps_dp[0].numpy(), eps_z=eps_z[0, :, :Ty].numpy().copy(),
                         w_ceil=attn.sum(0).numpy().astype(np.int32), idx=attn.argmax(1).numpy().astype(np.int32),
                         y_length=np.int64(Ty), wav=r["o"][0, 0].numpy())
-    print("tiny model: T_x", T, "T_y", Ty, "onnx bytes", os.path.getsize(path), "wav absmax %.3f" % float(r["o"].abs().max()))
+    print("tiny model: T_x", T, "T_y", Ty, "onnx bytes", onnx_bytes, "wav absmax %.3f" % float(r["o"].abs().max()))
 
 
 if __name__ == "__main__":

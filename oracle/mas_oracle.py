@@ -2,9 +2,9 @@
 (training/vits2/monotonic_align/core.pyx:7-34, driver monotonic_align/__init__.py:6-22).  TEST INFRASTRUCTURE: only tests/,
 __graft_entry__.smoke() and bench.py's CPU legs may import this; the product path is vosk_tts_b200/csrc (mas_kernel).
 
-Pinned against the reference itself: oracle/build_ref_mas.py compiles the reference's own core.pyx into oracle/_ref/ and
-tests/test_mas.py compares this restatement with it bit for bit on random cases (when oracle/_ref is present) and with the
-committed fixtures tests/golden/mas_*.npz that oracle/make_golden_mas.py generated from it.
+Pinned against the reference itself: oracle/build_ref_mas.py compiles the reference's own core.pyx into oracle/_ref/, and
+tests/test_mas.py compares this restatement bit for bit with the committed fixtures tests/golden/mas_*.npz that
+oracle/make_golden_mas.py and oracle/make_golden_reference.py generated from it.
 """
 import numpy as np
 

@@ -1,31 +1,24 @@
 """SURVEY.md section 8f rank 3: the other inverse-STFT decoders of the reference (Multistream_iSTFT_Generator,
-iSTFT_Generator).  The oracle restatement and the weight packing are pinned against the UNMODIFIED reference on CPU
-(build container only); the CUDA engine's parity run for them is tests/test_gpu_parity.py::test_istft_decoder_variants_vs_oracle."""
-import copy
+iSTFT_Generator).  The oracle restatement and the weight packing are pinned on CPU against what the UNMODIFIED reference
+computed and exported (tests/golden/decoder_variants.npz, *_model_onnx.npz, written by oracle/make_golden_reference.py);
+the CUDA engine's parity run for them is tests/test_gpu_parity.py::test_istft_decoder_variants_vs_oracle."""
+import json
+import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import ref_harness as rh
+from conftest import GOLDEN
+from oracle import onnx_fixture
 from oracle import vits_oracle as vo
+from oracle.make_golden_reference import VARIANT_SEED, VARIANT_T, VARIANT_VOCAB as N_VOCAB, variant_inputs, variant_training_json
 from vosk_tts_b200 import config as C, synthetic, weights
-
-pytestmark = pytest.mark.skipif(not rh.available(), reason="needs the reference tree")
-
-N_VOCAB = 40
 
 
 def _training_json(flag):
-    j = copy.deepcopy(rh.load_ref_config())
-    m = j["model"]
-    m.update(inter_channels=64, hidden_channels=64, filter_channels=128, n_heads=2, n_layers=3, kernel_size=3,
-             resblock_kernel_sizes=[3, 5], resblock_dilation_sizes=[[1, 3, 5], [1, 3, 5]], upsample_rates=[4, 4],
-             upsample_initial_channel=64, upsample_kernel_sizes=[16, 16], gin_channels=32,
-             mb_istft_vits=False, ms_istft_vits=False, istft_vits=False)
-    m[flag] = True
-    j["data"]["n_speakers"] = 4
-    return j
+    with open(os.path.join(GOLDEN, "reference_config.json")) as f:
+        return variant_training_json(json.load(f), flag)
 
 
 @pytest.mark.parametrize("flag,kind", [("ms_istft_vits", "ms_istft"), ("istft_vits", "istft"), ("mb_istft_vits", "mb_istft")])
@@ -33,24 +26,19 @@ def test_oracle_matches_reference_for_decoder_variant(flag, kind):
     tj = _training_json(flag)
     cfg = C.from_training_json(tj, n_vocab=N_VOCAB)
     assert cfg["decoder"] == kind and C.hop_total(cfg) == (64 if kind == "istft" else 256)
-    sd = synthetic.make_random_checkpoint(cfg, 11)
-    net = rh.build_reference_model(sd, cfg=tj, n_vocab=N_VOCAB)
-    folded = weights.fold_weight_norm(sd)
-    g = torch.Generator().manual_seed(3)
-    T = 19
-    tok = torch.randint(0, N_VOCAB, (1, T), generator=g)
-    eps_dp = torch.randn(1, 2, T, generator=g)
-    eps_z = torch.randn(1, cfg["inter_channels"], 400 * T, generator=g)     # the random SDP of this seed is slow-spoken
+    folded = weights.fold_weight_norm(synthetic.make_random_checkpoint(cfg, VARIANT_SEED))
+    tok, eps_dp, eps_z = variant_inputs(cfg)
+    T = VARIANT_T
     scales = [0.8, 1.0, 0.8]
     torch.set_num_threads(1)
-    r = rh.reference_infer(net, tok, torch.tensor([T]), torch.tensor([2]), scales, eps_dp, lambda s: eps_z[:, :, :s[2]])
     with torch.no_grad():
         o = vo.infer(folded, cfg, tok, torch.tensor([T]), torch.tensor([2]), scales, eps_dp, eps_z, return_all=True)
-    attn = r["attn"][0, 0]
-    assert np.array_equal(o["w_ceil"][0, 0].numpy().astype(np.int32), attn.sum(0).numpy().astype(np.int32))
-    assert np.array_equal(o["idx"][0].numpy(), attn.argmax(1).numpy())
-    assert o["o"].shape == r["o"].shape and r["o"].shape[-1] == int(o["y_lengths"][0]) * C.hop_total(cfg)
-    assert float((o["o"] - r["o"]).abs().max()) < 1e-5
+    ref = np.load(os.path.join(GOLDEN, "decoder_variants.npz"))
+    assert np.array_equal(o["w_ceil"][0, 0].numpy().astype(np.int32), ref[kind + "_w_ceil"])
+    assert np.array_equal(o["idx"][0].numpy(), ref[kind + "_idx"])
+    wav = o["o"][0, 0].numpy()
+    assert o["o"].shape[:2] == (1, 1) and wav.size == int(ref[kind + "_wav_length"]) == int(o["y_lengths"][0]) * C.hop_total(cfg)
+    assert float(np.abs(wav[ref[kind + "_wav_idx"]] - ref[kind + "_wav_val"]).max()) < 1e-5
 
 
 @pytest.mark.parametrize("flag", ["ms_istft_vits", "istft_vits"])
@@ -58,7 +46,7 @@ def test_packed_tail_filter_is_what_the_decoder_applies(flag):
     """pack() hands the CUDA tail kernel one 63-tap filter per band: the learned multistream filter, or a unit impulse."""
     tj = _training_json(flag)
     cfg = C.from_training_json(tj, n_vocab=N_VOCAB)
-    folded = weights.fold_weight_norm(synthetic.make_random_checkpoint(cfg, 11))
+    folded = weights.fold_weight_norm(synthetic.make_random_checkpoint(cfg, VARIANT_SEED))
     blob, man = weights.pack(folded, cfg, tc=False)
     ent = {}
     for line in man.strip().splitlines():
@@ -89,10 +77,9 @@ def test_variant_is_recognised_in_an_exported_graph(flag, kind, tmp_path):
     from vosk_tts_b200 import onnx_weights as ow
     tj = _training_json(flag)
     cfg = C.from_training_json(tj, n_vocab=N_VOCAB)
-    net = rh.build_reference_model(synthetic.make_random_checkpoint(cfg, 11), cfg=tj, n_vocab=N_VOCAB)
-    path = rh.export_reference_onnx(tmp_path / "model.onnx", net, n_vocab=N_VOCAB)
-    got = ow.config_from_onnx(str(path))
+    path, _ = onnx_fixture.unpack(os.path.join(GOLDEN, kind + "_model_onnx.npz"), str(tmp_path / "model.onnx"))
+    got = ow.config_from_onnx(path)
     assert got == cfg
-    blob, man = weights.pack(ow.state_dict_from_onnx(str(path)), got, tc=False)
-    b2, m2 = weights.pack(weights.fold_weight_norm(synthetic.make_random_checkpoint(cfg, 11)), cfg, tc=False)
+    blob, man = weights.pack(ow.state_dict_from_onnx(path), got, tc=False)
+    b2, m2 = weights.pack(weights.fold_weight_norm(synthetic.make_random_checkpoint(cfg, VARIANT_SEED)), cfg, tc=False)
     assert man == m2 and float(np.abs(blob - b2).max()) < 1e-6

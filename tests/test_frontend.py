@@ -68,24 +68,16 @@ def test_missing_model_is_an_error_not_a_download():
         Model(model_name="vosk-model-tts-ru-0.9-multi")
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/vosk_tts/g2p.py"), reason="reference tree absent")
 def test_g2p_matches_reference_converter():
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_g2p", "/root/reference/vosk_tts/g2p.py")
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    import itertools
-    words = ["прив+ет", "абстр+акция", "+ёлка", "подъ+езд", "семь+я", "чащ+а", "й+од", "объявл+ение", "в+ьюга", "съ+ёмка",
-             "по-р+усски", "+я", "мышь", "компь+ютер", "ш+ёлк", "Гог+оль"]
-    letters = "абвгдеёжзийклмнопрстуфхцчшщъыьэюя"
-    rng = np.random.RandomState(0)
-    for _ in range(300):
-        n = rng.randint(1, 9)
-        w = "".join(letters[i] for i in rng.randint(0, len(letters), n))
-        p = rng.randint(0, n)
-        words.append(w[:p] + "+" + w[p:])
-    for w in words:
-        assert g2p.convert(w) == ref.convert(w), w
+    """vosk_tts.g2p.convert of the reference on hand-picked and seeded random stressed words (tests/golden/g2p_reference.json,
+    written by oracle/make_golden_reference.py)."""
+    from oracle.make_golden_reference import g2p_words
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "g2p_reference.json"), encoding="utf-8") as f:
+        ref = json.load(f)
+    words = g2p_words()
+    assert [w for w, _ in ref] == words and len(words) == 316
+    for w, want in ref:
+        assert g2p.convert(w) == want, w
 
 
 class _StubEngine:

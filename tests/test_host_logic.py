@@ -106,9 +106,8 @@ def test_convt_polyphase_equals_conv_transpose(u, K):
 
 
 def test_config_mapping_from_reference_json():
-    path = "/root/reference/training/vits2/configs/mb_istft_vits2_multi.json"
-    if not os.path.exists(path):
-        pytest.skip("reference tree absent")
+    """The reference's training/vits2/configs/mb_istft_vits2_multi.json (tests/golden/reference_config.json)."""
+    path = os.path.join(ROOT, "tests", "golden", "reference_config.json")
     assert C.from_training_json(path) == C.DEFAULT_CONFIG
     assert C.hop_total(C.DEFAULT_CONFIG) == 256
 

@@ -1,8 +1,6 @@
 """Monotonic Alignment Search: oracle (numpy restatement of training/vits2/monotonic_align/core.pyx) against fixtures generated
 by the reference's own compiled Cython kernel (oracle/make_golden_mas.py), and the CUDA kernel (csrc/mas.cuh, through the C ABI)
 against both -- bit-exact, it is integer/index work."""
-import glob
-import importlib.util
 import os
 import sys
 
@@ -13,6 +11,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import mas_oracle as O  # noqa: E402
 from oracle.make_golden_mas import LARGE, large_case  # noqa: E402
+from oracle.make_golden_reference import mas_trials  # noqa: E402
 
 G = np.load(os.path.join(ROOT, "tests", "golden", "mas_cases.npz"))
 
@@ -52,26 +51,13 @@ def test_oracle_matches_reference_fixtures():
 
 
 def test_oracle_matches_compiled_reference_when_present():
-    so = glob.glob(os.path.join(ROOT, "oracle", "_ref", "ref_mas_core*.so"))
-    if not so:
-        pytest.skip("oracle/_ref not built (python oracle/build_ref_mas.py; needs /root/reference)")
-    spec = importlib.util.spec_from_file_location("ref_mas_core", so[0])
-    try:
-        ref = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(ref)
-    except ImportError as ex:
-        pytest.skip("oracle/_ref not loadable with this interpreter: %s" % ex)
-    rng = np.random.RandomState(3)
-    for trial in range(40):
-        B, Ty, Tx = rng.randint(1, 4), rng.randint(1, 80), rng.randint(1, 30)
-        nc = (rng.randn(B, Ty, Tx) * 3).astype(np.float32)
-        if trial % 4 == 0:
-            nc = np.round(nc)                                   # ties
-        ty = np.array([rng.randint(1, Ty + 1) for _ in range(B)], np.int32)
-        tx = np.array([rng.randint(1, min(Tx, t) + 1) for t in ty], np.int32)
-        v, p = nc.copy(), np.zeros(nc.shape, np.int32)
-        ref.maximum_path_c(p, v, ty, tx)
-        assert np.array_equal(O.maximum_path(nc, ty, tx), p)
+    """40 random ragged trials (every fourth with ties) against the paths the reference's compiled maximum_path_c returned
+    (tests/golden/mas_reference_trials.npz, written by oracle/make_golden_reference.py)."""
+    ref = np.load(os.path.join(ROOT, "tests", "golden", "mas_reference_trials.npz"))
+    trials = list(mas_trials())
+    assert len(trials) == len(ref.files) == 40
+    for i, (nc, ty, tx) in enumerate(trials):
+        assert np.array_equal(O.maximum_path(nc, ty, tx), ref["t%d_path" % i]), i
 
 
 def test_abi_exports_mas():

@@ -1,29 +1,23 @@
 """Weights and configuration straight from a ``model.onnx`` written by the reference's own export path
-(training/vits2/onnx_export.py:60-104, run here on the seeded reference model; build container only)."""
+(training/vits2/onnx_export.py:60-104, run on the seeded reference model; stored as tests/golden/*_onnx.npz by
+oracle/make_golden_reference.py and oracle/make_tiny_onnx.py, see oracle/onnx_fixture.py)."""
 import os
-import time
 
 import numpy as np
 import pytest
 
-from oracle import ref_harness as rh
+from oracle import onnx_fixture
 from vosk_tts_b200 import config as C, onnx_weights as ow, synthetic, weights
 
-needs_ref = pytest.mark.skipif(not rh.available(), reason="needs the reference tree to export model.onnx")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 @pytest.fixture(scope="module")
 def onnx_path(tmp_path_factory):
-    if not rh.available():
-        pytest.skip("needs the reference tree")
-    sd = synthetic.make_random_checkpoint(C.DEFAULT_CONFIG, 1234)
-    net = rh.build_reference_model(sd)
-    path = tmp_path_factory.mktemp("onnx") / "model.onnx"
-    rh.export_reference_onnx(path, net)
-    return str(path)
+    """model.onnx of the full-size model from the seed-1234 synthetic checkpoint."""
+    return onnx_fixture.unpack(os.path.join(GOLDEN, "model_onnx.npz"), str(tmp_path_factory.mktemp("onnx") / "model.onnx"))[0]
 
 
-@needs_ref
 def test_state_dict_from_onnx_matches_folded_checkpoint(onnx_path):
     sd = ow.state_dict_from_onnx(onnx_path)
     ref = weights.fold_weight_norm(synthetic.make_random_checkpoint(C.DEFAULT_CONFIG, 1234))
@@ -42,13 +36,11 @@ def test_state_dict_from_onnx_matches_folded_checkpoint(onnx_path):
     assert sd["dp.flows.0.logs"].shape == (2, 1)
 
 
-@needs_ref
 def test_config_from_onnx_recovers_the_training_configuration(onnx_path):
     cfg = ow.config_from_onnx(onnx_path)
     assert cfg == C.DEFAULT_CONFIG
 
 
-@needs_ref
 def test_packed_blob_from_onnx_has_the_same_layout(onnx_path):
     sd = ow.state_dict_from_onnx(onnx_path)
     cfg = ow.config_from_onnx(onnx_path)
@@ -65,17 +57,19 @@ def test_reader_rejects_non_onnx(tmp_path):
         ow.read_graph(str(p))
 
 
-# ---- committed fixture (tests/golden/tiny_model.onnx + tiny_onnx.npz, oracle/make_tiny_onnx.py): runs without the reference
-TINY = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "tiny_model.onnx")
+# ---- reduced-width model (tests/golden/tiny_model_onnx.npz + tiny_onnx.npz, oracle/make_tiny_onnx.py)
+@pytest.fixture(scope="module")
+def tiny_path(tmp_path_factory):
+    return onnx_fixture.unpack(os.path.join(GOLDEN, "tiny_model_onnx.npz"), str(tmp_path_factory.mktemp("tiny") / "model.onnx"))[0]
 
 
-def _tiny():
-    g = np.load(os.path.join(os.path.dirname(TINY), "tiny_onnx.npz"))
-    return ow.state_dict_from_onnx(TINY), ow.config_from_onnx(TINY), g
+def _tiny(path):
+    g = np.load(os.path.join(GOLDEN, "tiny_onnx.npz"))
+    return ow.state_dict_from_onnx(path), ow.config_from_onnx(path), g
 
 
-def test_tiny_onnx_config_is_recovered():
-    cfg = ow.config_from_onnx(TINY)
+def test_tiny_onnx_config_is_recovered(tiny_path):
+    cfg = ow.config_from_onnx(tiny_path)
     assert (cfg["hidden_channels"], cfg["inter_channels"], cfg["filter_channels"], cfg["n_layers"], cfg["n_heads"]) == (64, 64, 128, 3, 2)
     assert (cfg["n_vocab"], cfg["n_speakers"], cfg["gin_channels"]) == (40, 4, 32)
     assert cfg["resblock_kernel_sizes"] == [3, 5] and cfg["resblock_dilation_sizes"] == [[1, 3, 5], [1, 3, 5]]
@@ -85,11 +79,11 @@ def test_tiny_onnx_config_is_recovered():
     assert (cfg["flow_n_flows"], cfg["flow_wn_layers"], cfg["flow_kernel_size"]) == (4, 4, 5)
 
 
-def test_oracle_on_onnx_weights_reproduces_the_reference_output():
+def test_oracle_on_onnx_weights_reproduces_the_reference_output(tiny_path):
     """model.onnx initializers -> oracle == the waveform the reference produced from the same module (CPU)."""
     import torch
     from oracle import vits_oracle as vo
-    sd, cfg, g = _tiny()
+    sd, cfg, g = _tiny(tiny_path)
     w = {k: torch.from_numpy(np.array(v)) for k, v in sd.items()}
     tok = torch.as_tensor(g["tokens"])[None]
     T = tok.shape[1]
@@ -103,9 +97,9 @@ def test_oracle_on_onnx_weights_reproduces_the_reference_output():
     assert np.abs(o["o"][0, 0].numpy() - g["wav"]).max() < 1e-5
 
 
-def test_session_packing_accepts_the_numpy_state_dict():
+def test_session_packing_accepts_the_numpy_state_dict(tiny_path):
     """VitsSession folds + packs whatever Model hands it; for model.onnx that is a dict of numpy arrays."""
-    sd, cfg, _ = _tiny()
+    sd, cfg, _ = _tiny(tiny_path)
     folded = weights.fold_weight_norm(sd)
     assert not weights.tc_supported(cfg)
     blob, man = weights.pack(folded, cfg)
@@ -114,14 +108,14 @@ def test_session_packing_accepts_the_numpy_state_dict():
 
 
 @pytest.mark.gpu
-def test_engine_from_onnx_initializers_reproduces_the_reference_output():
+def test_engine_from_onnx_initializers_reproduces_the_reference_output(tiny_path):
     """The deployment path end to end on the GPU: model.onnx -> initializers -> packed weights -> CUDA engine (fp32 mode:
     the reduced-width fixture has 64/32/16-channel convs, below the 64-multiple the tensor-core path packs)."""
     import torch
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
     from vosk_tts_b200.engine import Engine
-    sd, cfg, g = _tiny()
+    sd, cfg, g = _tiny(tiny_path)
     blob, man = weights.pack(sd, cfg, tc=False)
     e = Engine(cfg, blob, man, device=0, precision=0)
     try:
@@ -137,7 +131,7 @@ def test_engine_from_onnx_initializers_reproduces_the_reference_output():
 
 
 @pytest.mark.gpu
-def test_model_directory_in_deployed_layout_synthesizes(tmp_path):
+def test_model_directory_in_deployed_layout_synthesizes(tmp_path, tiny_path):
     """What a vosk-tts user has on disk -- model.onnx + config.json + dictionary (vosk_tts/model.py:40-55) -- is all that
     `Model` / `Synth` need: text in, 22.05 kHz 16-bit WAV out, no checkpoint, no training json."""
     import json
@@ -153,7 +147,7 @@ def test_model_directory_in_deployed_layout_synthesizes(tmp_path):
            "model_type": "vits", "audio": {"sample_rate": 22050}}
     (tmp_path / "config.json").write_text(json.dumps(cfg), encoding="utf-8")
     (tmp_path / "dictionary").write_text("привет 1.0 p rj i0 vj e1 t\n", encoding="utf-8")
-    shutil.copy(TINY, tmp_path / "model.onnx")
+    shutil.copy(tiny_path, tmp_path / "model.onnx")
     m = Model(model_path=tmp_path)
     assert m.onnx.cfg["hidden_channels"] == 64 and m.onnx.cfg["n_speakers"] == 4
     s = Synth(m)

@@ -1,7 +1,6 @@
 """gRPC service (vosk_tts_b200/server.py) against the wire contract of the reference's server/tts_service.proto.
 CPU tests use a stub Synth; the GPU test serves the real engine (tiny exported model) to concurrent clients."""
 import json
-import shutil
 import threading
 from pathlib import Path
 
@@ -119,7 +118,8 @@ def test_real_engine_behind_the_service(tmp_path):
            "model_type": "vits", "audio": {"sample_rate": 22050}}
     (tmp_path / "config.json").write_text(json.dumps(cfg), encoding="utf-8")
     (tmp_path / "dictionary").write_text("привет 1.0 p rj i0 vj e1 t\nмир 1.0 m i1 r\n", encoding="utf-8")
-    shutil.copy(Path(__file__).parent / "golden" / "tiny_model.onnx", tmp_path / "model.onnx")
+    from oracle import onnx_fixture
+    onnx_fixture.unpack(str(Path(__file__).parent / "golden" / "tiny_model_onnx.npz"), str(tmp_path / "model.onnx"))
     synth = Synth(Model(model_path=tmp_path))
     srv, port = S.make_server(synth, "127.0.0.1:0", threads=3, chunk_frames=8)
     srv.start()
